@@ -377,9 +377,37 @@ class Ctx:
     pass
 
 
-def measure(cx, wl: str, steps: int, warmup: int, *, cpu_budget_s: float = 0.0, e2e_cap_units: int = 1 << 24):
+DUMP_UNITS = 1 << 16                     # --dump-outputs: output units kept per workload (a fixed sample of larger outputs)
+DUMP_WORD = {"sha256": "<u4", "sha256_2p30": "<u4", "aes": "u1", "crc16": "<u2", "gemm": "<f4"}
+DUMP_MAX_BYTES = 64 << 20
+
+
+def output_sample(torch, out, n: int, unit_base: int, wl: str):
+    """The voted output of one launch as its caller reads it, for --dump-outputs: at most DUMP_UNITS units, drawn with a
+    fixed seed so that two runs with the same arguments sample the same units.  One row per unit, one column per output
+    word (digest word, byte, crc or fp32 element), widened exactly to float64 (u32 words) or float32.  Returns
+    (values, global unit indices as float64)."""
+    import numpy as np
+    k = min(n, DUMP_UNITS)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False)) if k < n else np.arange(n)
+    rows = out.view(torch.uint8)[: n * OUT_B[wl]].view(n, OUT_B[wl])[torch.from_numpy(idx).to(out.device)]
+    vals = rows.cpu().numpy().view(DUMP_WORD[wl])
+    return vals.astype(np.float64 if DUMP_WORD[wl] == "<u4" else np.float32), (unit_base + idx).astype(np.float64)
+
+
+def write_dump(path: str, arrays: dict) -> None:
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}"
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def measure(cx, wl: str, steps: int, warmup: int, *, cpu_budget_s: float = 0.0, e2e_cap_units: int = 1 << 24, dump=None):
     """One workload on this rank's GPU: device-timed region, single-launch loop, end-to-end host call.  Returns the
-    JSON-line dict on rank 0 (None elsewhere).  Every rank must call it with the same arguments."""
+    JSON-line dict on rank 0 (None elsewhere).  Every rank must call it with the same arguments.  With a `dump` dict,
+    rank 0 adds to it a sample of the output of the last timed step (`<wl>`, `<wl>_units`) and the counters its
+    coast_sync() returned after the timed region (`<wl>_counters`)."""
     torch, cb, rt, dist = cx.torch, cx.cb, cx.rt, cx.dist
     world, rank, dev = cx.world, cx.rank, cx.dev
     from coast_b200.shard import shard_range
@@ -490,6 +518,8 @@ def measure(cx, wl: str, steps: int, warmup: int, *, cpu_budget_s: float = 0.0, 
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
     timed_launches = launches
+    if dump is not None and rank == 0 and descs:
+        dump[wl], dump[wl + "_units"] = output_sample(torch, outs[(steps - 1) % nsets], n, unit_base, wl)
     # the SM clock the region REALLY ran at: cycles / nanoseconds between the two probes, per SM that answered both, median
     p0, p1 = probe0.view(-1, 2).cpu(), probe1.view(-1, 2).cpu()
     both = (p0[:, 1] > 0) & (p1[:, 1] > p0[:, 1])
@@ -509,6 +539,9 @@ def measure(cx, wl: str, steps: int, warmup: int, *, cpu_budget_s: float = 0.0, 
             rt.counters_detach()                           # the single-launch loop and the host calls below tally locally again
     else:
         n_counted = n
+    if dump is not None and rank == 0:
+        import numpy as np
+        dump[wl + "_counters"] = np.array(list(st.as_dict().values()), dtype=np.float64)
     if wl.startswith("sha256"):
         assert st.errors_corrected == 0 and st.syncs == 32 * n_counted * (steps + warmup), (st, n_counted)
     if wl == "aes" and (rank == 0 or not peer_fold):
@@ -755,14 +788,15 @@ def run_ours(args):
                                                       log=lambda m: print("bench: " + m, file=sys.stderr))
 
     main_cpu = 0.0 if args.no_cpu_baseline else 10.0
-    line = measure(cx, args.workload, args.steps, args.warmup, cpu_budget_s=main_cpu)
+    dump = {} if args.dump_outputs else None
+    line = measure(cx, args.workload, args.steps, args.warmup, cpu_budget_s=main_cpu, dump=dump)
     if args.workload == "sha256" and not args.no_also:
         also = {}
         wls = ["aes", "gemm", "crc16", "sha256_2p30"] if cx.world == 1 else ["sha256_2p30", "gemm"]
         for wl in wls:
             t0 = time.perf_counter()
             try:
-                sub = measure(cx, wl, ALSO_STEPS[wl], 3, cpu_budget_s=0.0 if args.no_cpu_baseline else 3.0)
+                sub = measure(cx, wl, ALSO_STEPS[wl], 3, cpu_budget_s=0.0 if args.no_cpu_baseline else 3.0, dump=dump)
             except Exception as exc:                       # an extra workload must never cost the headline line
                 sub = {"error": repr(exc)[:300]}
                 if cx.dist is not None:
@@ -778,6 +812,8 @@ def run_ours(args):
         if line is not None:
             line["also"] = also
     if cx.rank == 0:
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if cx.dist is not None:
         cx.dist.barrier()
@@ -797,7 +833,15 @@ def main():
     ap.add_argument("--threads", type=int, default=0, help="--impl reference: host threads (default: all; config 1 is 1 thread)")
     ap.add_argument("--workload", choices=["sha256", "sha256_2p30", "aes", "crc16", "gemm"], default="sha256",
                     help="default sha256 = BASELINE configs[1], the headline line (with the other configs under `also`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of each timed workload's last-step output, and its counters, as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "ours":
+            ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

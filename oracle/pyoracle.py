@@ -193,14 +193,6 @@ def chstone_site_of_input_bit(byte: int, bit: int):
     return 421 * (byte // 64) + (byte % 64) // 4, 8 * (byte % 4) + bit
 
 
-def chstone_indata() -> np.ndarray:
-    """The benchmark's own 2 x 8192-byte input, read out of oracle/_ref/libref_chsha.so (compiled reference data)."""
-    r = ref("chsha")
-    r.ref_chsha_indata.restype = C.c_void_p
-    n = int(r.ref_chsha_len())
-    return np.frombuffer((C.c_uint8 * n).from_address(r.ref_chsha_indata()), dtype=np.uint8).copy()
-
-
 def aes128(state: bytes, key: bytes, direction: int):
     s = np.frombuffer(state, dtype=np.uint8).copy()
     k = np.frombuffer(key, dtype=np.uint8).copy()

@@ -17,13 +17,17 @@ Contents
   mm      : mm_tmr.c 9x9 uint32 operands, results_matrix, xor_golden; matrixMultiply.c int operands/results
   chaes   : tests/chstone/aes: the benchmark's FIPS-197 vector through the reference's own encrypt()/decrypt(), 40 random
             (block, key) pairs both directions, DWC/TMR runs of the reference functions with a flipped input byte in one replica
-  chsha   : tests/chstone/sha: the golden outData of sha_driver.c (the 16 KiB indata itself is NOT copied: only its
-            SHA-256, the GPU test reads the bytes from oracle/_ref/libref_chsha.so), reference digests of Philox
-            streams of several lengths, and TMR/DWC runs with input flips
+  chsha   : tests/chstone/sha: the golden outData of sha_driver.c and the SHA-256 of its 16 KiB indata, reference
+            digests of Philox streams of several lengths, and TMR/DWC runs with input flips
   qsort   : tests/quicksort: the benchmark's own 580-int input (srand(0)) with the SHA-256 of what quick_sort() makes of it,
             and reference outputs for random arrays of several lengths (duplicates, extremes)
   xmr     : TMR/DWC runs of the reference functions with a single-bit flip in ONE replica's private
             copy of its input (the only fault sites reachable without editing reference sources)
+
+Next to it, data the tests would otherwise read out of the reference checkout:
+  chstone_sha_indata.bin : the 2 x 8192-byte input of tests/chstone/sha (sha_data.c), as the benchmark hashes it
+  reference_programs.json: the OPT_PASSES sweep of unittest/cfg/full.yml, and the scope facts (directives, definitions,
+                           calls) the BOARD=b200 pass reads out of tests/matrixMultiply and tests/sha256_common/sha256_tmr.c
 """
 import ctypes as C
 import json
@@ -318,6 +322,24 @@ def main():
     path = os.path.join(ROOT, "tests", "golden", "coast_golden.json")
     with open(path, "w") as f:
         json.dump(g, f, separators=(",", ":"))
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+    path = os.path.join(ROOT, "tests", "golden", "chstone_sha_indata.bin")
+    indata.tofile(path)
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+    import yaml
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    import build_reference_tests as brt
+    brt.build_all()
+    with open("/root/reference/unittest/cfg/full.yml") as f:
+        progs = {"full_yml_opt_passes": yaml.safe_load(f)["OPT_PASSES"], "scope_facts": {}}
+    for target in ("matrixMultiply", "sha256_tmr"):
+        with open(os.path.join(brt.OUT, target, target + ".scope")) as f:
+            progs["scope_facts"][target] = f.read()
+    path = os.path.join(ROOT, "tests", "golden", "reference_programs.json")
+    with open(path, "w") as f:
+        json.dump(progs, f, indent=1)
     print("wrote", path, os.path.getsize(path), "bytes")
 
 

@@ -50,6 +50,30 @@ def test_both_arms_print_the_same_config_object():
         assert bench.config_for(wl, 8)["parallelism"] == "shard8" and bench.config_for(wl, 8)["workload"] == bench.WORKLOAD_NAMES[wl]
 
 
+def test_dumped_output_sample_is_exact_seeded_and_bounded(tmp_path):
+    """--dump-outputs: the same units are sampled on every run, their words are widened without loss, and the files of
+    every workload together stay within the size bound."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    n = 3 * bench.DUMP_UNITS
+    out = torch.from_numpy(np.random.default_rng(1).integers(0, 256, n * 32, dtype=np.uint8))
+    vals, units = bench.output_sample(torch, out, n, 0, "sha256")
+    again, units2 = bench.output_sample(torch, out, n, 0, "sha256")
+    assert vals.dtype == np.float64 and vals.shape == (bench.DUMP_UNITS, 8) and np.array_equal(units, units2)
+    assert np.array_equal(vals, again)
+    assert np.array_equal(vals, out.numpy().view("<u4").reshape(n, 8)[units.astype(np.int64)])
+    c = torch.randn(100)
+    vals, units = bench.output_sample(torch, c, 100, 7, "gemm")
+    assert np.array_equal(vals[:, 0], c.numpy()) and units[0] == 7
+    words = {wl: bench.OUT_B[wl] // np.dtype(w).itemsize for wl, w in bench.DUMP_WORD.items()}
+    total = sum(bench.DUMP_UNITS * (words[wl] * (8 if w == "<u4" else 4) + 8) for wl, w in bench.DUMP_WORD.items())
+    assert total <= bench.DUMP_MAX_BYTES
+    bench.write_dump(str(tmp_path), {"gemm": vals})
+    assert np.array_equal(np.load(tmp_path / "gemm.npy"), vals)
+
+
 def test_reference_arm_reports_the_median_of_individually_timed_steps():
     res = _run(["--threads", "2", "--workload", "crc16"])
     d = json.loads([ln for ln in res.stdout.splitlines() if ln.startswith("{")][0])

@@ -13,7 +13,7 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
-from build_reference_tests import CASES, OUT, REF, exe_path, make_cmd  # noqa: E402  (the list the driver's build() uses too)
+from build_reference_tests import CASES, OUT, REF, exe_path, make_cmd, run_env  # noqa: E402  (the list build() uses too)
 
 
 @pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout absent (GPU box)")
@@ -59,7 +59,7 @@ def test_unchanged_reference_tests_run_on_the_gpu(tdir, target, extra, entry, re
     exe = exe_path(target, extra)
     if not os.path.exists(exe):
         pytest.skip("binary was not built on the CPU box (needs the reference checkout)")
-    res = subprocess.run([exe], capture_output=True, text=True, timeout=120)
+    res = subprocess.run([exe], capture_output=True, text=True, timeout=120, env=run_env())
     assert res.returncode == rc, res.stdout + res.stderr          # unittest.py:76-78: non-zero exit = fail
     assert re.search(regex, res.stdout), res.stdout + res.stderr   # unittest.py:80-86 regex on stdout
 
@@ -79,11 +79,11 @@ FULL_YML_SWEEP = [
 ]
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/unittest/cfg/full.yml"), reason="reference checkout absent (GPU box)")
 def test_sweep_list_is_the_reference_one():
-    import yaml
-    cfg = yaml.safe_load(open("/root/reference/unittest/cfg/full.yml"))
-    assert cfg["OPT_PASSES"] == FULL_YML_SWEEP
+    """the OPT_PASSES of the reference's unittest/cfg/full.yml, stored by tests/golden/make_golden.py"""
+    import json
+    with open(os.path.join(ROOT, "tests", "golden", "reference_programs.json")) as f:
+        assert json.load(f)["full_yml_opt_passes"] == FULL_YML_SWEEP
 
 
 def test_every_sweep_entry_parses_without_an_ignored_token(built_lib):
@@ -118,7 +118,7 @@ def test_unittest_full_yml_sweep_on_the_gpu(target, regex):
     seen = {}
     for passes in FULL_YML_SWEEP:
         count = " -countErrors -countSyncs" if "-TMR" in passes else ""
-        env = dict(os.environ, COAST_OPT_PASSES_OVERRIDE=passes + count + " -verbose", COAST_REPORT_COUNTERS="1")
+        env = run_env(COAST_OPT_PASSES_OVERRIDE=passes + count + " -verbose", COAST_REPORT_COUNTERS="1")
         res = subprocess.run([exe], capture_output=True, text=True, timeout=120, env=env)
         assert res.returncode == 0, (passes, res.stdout + res.stderr)
         assert re.search(regex, res.stdout), (passes, res.stdout + res.stderr)
@@ -145,6 +145,6 @@ def test_strict_flags_turn_an_unhonoured_flag_into_an_error():
     exe = os.path.join(OUT, "aes", "aes.out")
     if not os.path.exists(exe):
         pytest.skip("binary was not built on the CPU box (needs the reference checkout)")
-    env = dict(os.environ, COAST_OPT_PASSES_OVERRIDE="-TMR -noMemReplication", COAST_STRICT_FLAGS="1")
+    env = run_env(COAST_OPT_PASSES_OVERRIDE="-TMR -noMemReplication", COAST_STRICT_FLAGS="1")
     res = subprocess.run([exe], capture_output=True, text=True, timeout=120, env=env)
     assert res.returncode != 0 and "has no in-loop store votes" in res.stderr

@@ -5,6 +5,7 @@ through the C ABI and through the unchanged benchmark built by the BOARD=b200 fl
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -150,11 +151,13 @@ def test_chaes_entry_point_and_host_call(rt, oracle, golden):
 
 @pytest.mark.gpu
 def test_unchanged_chstone_aes_benchmark_runs_on_the_gpu():
+    sys.path.insert(0, os.path.join(ROOT, "tools"))
+    from build_reference_tests import run_env
     exe = os.path.join(ROOT, "oracle", "_ref", "b200", "chstone_aes", "aes.out")
     if not os.path.exists(exe):
         pytest.skip("binary was not built on the CPU box (needs the reference checkout)")
     for passes in ("-TMR", "-DWC", ""):
-        res = subprocess.run([exe], capture_output=True, text=True, timeout=120, env=dict(os.environ, COAST_OPT_PASSES_OVERRIDE=passes + " -verbose"))
+        res = subprocess.run([exe], capture_output=True, text=True, timeout=120, env=run_env(COAST_OPT_PASSES_OVERRIDE=passes + " -verbose"))
         assert res.returncode == 0, res.stdout + res.stderr
         assert re.search(r"encrypted message \t3925841d02dc09fbdc118597196a0b32\ndecrypto message\t3243f6a8885a308d313198a2e0370734RESULT: PASS", res.stdout)
         assert ("xmr_chaes_enc_nc%d" % (3 if "TMR" in passes else 2 if "DWC" in passes else 1)) in res.stderr and "xmr_chaes_dec_" in res.stderr

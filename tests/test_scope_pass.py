@@ -4,11 +4,10 @@ own directives, calls are redirected only for functions that are IN it and have 
 function on the CPU, and an explicit __xMR that cannot be honoured fails the build naming the function.
 The programs below are this repo's own (written for the test), built in a temp directory with the same Makefile contract
 as the reference's test directories.  No GPU: the cases that run a binary are the ones whose protected region stays on the CPU."""
+import json
 import os
 import re
 import subprocess
-
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LEVEL = os.path.join(ROOT, "include")
@@ -89,16 +88,21 @@ def test_an_xmr_wrapper_around_a_kernel_entry_is_accepted_and_reported(tmp_path,
     assert "wrapper   run_test runs on the host; its protected work is the kernel entry it calls (__xMR)" in res.stdout and redirected(out)
 
 
-def scan(src):
-    tool = "/tmp/coast_scope_test"
+def scope_tool(tmp_path):
+    tool = str(tmp_path / "coast_scope")
     subprocess.run(["gcc", "-O1", "-o", tool, os.path.join(LEVEL, "makefiles", "coast_scope.c")], check=True)
+    return tool
+
+
+def scan(tmp_path, src):
+    tool = scope_tool(tmp_path)
     pre = subprocess.run(["gcc", "-E", "-w", "-DCOAST_SCOPE_SCAN", "-include", os.path.join(LEVEL, "coast_shim.h"), "-I", LEVEL, "-x", "c", "-"],
                          input=src, capture_output=True, text=True, check=True).stdout
     return subprocess.run([tool, "scan"], input=pre, capture_output=True, text=True, check=True).stdout.splitlines()
 
 
-def test_scanner_reads_directives_in_every_position_the_reference_tests_use():
-    facts = scan(r'''
+def test_scanner_reads_directives_in_every_position_the_reference_tests_use(tmp_path):
+    facts = scan(tmp_path, r'''
     __DEFAULT_NO_xMR
     unsigned __xMR results[9][9] = { {1, 2}, {3} };  unsigned __NO_xMR golden[9][9];
     struct S { int a; } __xMR sv;
@@ -118,17 +122,25 @@ def test_scanner_reads_directives_in_every_position_the_reference_tests_use():
     assert not [f for f in facts if "fp_t" in f]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tests"), reason="reference checkout absent (GPU box)")
-def test_the_reference_tests_get_the_scope_their_directives_ask_for(built_lib):
+def test_the_reference_tests_get_the_scope_their_directives_ask_for(tmp_path):
     """matrixMultiply.c: `int checkGolden() __NO_xMR` stays on the CPU, matrix_multiply (default scope) is offloaded, the explicitly
-    __xMR `initialize()` is reported as unprotected; sha256_tmr.c: __DEFAULT_NO_xMR + `void __xMR sha256_hash`"""
-    for tdir, extra, wants in (
-        ("matrixMultiply", [], ["offload   matrix_multiply -> coast_xmr_matrix_multiply   (default scope)", "WARNING   initialize is marked __xMR"]),
-        ("sha256_common", ["SRCFILES=/root/reference/tests/sha256_common/sha256_tmr.c"],
+    __xMR `initialize()` is reported as unprotected; sha256_tmr.c: __DEFAULT_NO_xMR + `void __xMR sha256_hash`.
+    The scope facts the scanner reads out of those two programs are stored in tests/golden/reference_programs.json
+    (tests/golden/make_golden.py); the pass decides from them as the make flow would, with each program's own -verbose."""
+    with open(os.path.join(ROOT, "tests", "golden", "reference_programs.json")) as f:
+        facts = json.load(f)["scope_facts"]
+    tool = scope_tool(tmp_path)
+    for target, verbose, wants in (
+        ("matrixMultiply", "0", ["offload   matrix_multiply -> coast_xmr_matrix_multiply   (default scope)", "WARNING   initialize is marked __xMR"]),
+        ("sha256_tmr", "1",
          ["scope: default no_xMR", "offload   sha256_hash -> coast_xmr_sha256_hash   (__xMR)", "inside    sha256_transform", "wrapper   sha_run_test",
           "WARNING   checkGolden is marked __xMR", "cpu-only  main"]),
     ):
-        res = subprocess.run(["make", "-B", "-C", f"/root/reference/tests/{tdir}", f"LEVEL={LEVEL}", "BOARD=b200"] + extra + ["exe"], capture_output=True, text=True)
+        scope = tmp_path / f"{target}.scope"
+        scope.write_text(facts[target])
+        res = subprocess.run([tool, "plan", os.path.join(LEVEL, "makefiles", "coast_entries.tab"), str(tmp_path / f"{target}.sed"),
+                              "checkGolden initialize", verbose, str(scope)], capture_output=True, text=True)
         assert res.returncode == 0, res.stdout + res.stderr
         for w in wants:
             assert w in res.stdout, (w, res.stdout)
+        assert "coast_xmr_" in (tmp_path / f"{target}.sed").read_text()

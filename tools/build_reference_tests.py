@@ -26,6 +26,15 @@ CASES = [
 ]
 
 
+def run_env(**extra) -> dict:
+    """Environment that runs a built program against THIS tree's coast_b200/libcoast_rt.so.  The programs' rpath is relative
+    to $ORIGIN, which the loader takes from the executable's resolved path: when oracle/_ref reaches the tree through a
+    link (or a copy made elsewhere), that path lies outside the tree.  LD_LIBRARY_PATH is searched before the rpath."""
+    env = dict(os.environ, **extra)
+    env["LD_LIBRARY_PATH"] = os.pathsep.join(p for p in (os.path.join(ROOT, "coast_b200"), os.environ.get("LD_LIBRARY_PATH")) if p)
+    return env
+
+
 def available() -> bool:
     return os.path.isdir(REF)
 
