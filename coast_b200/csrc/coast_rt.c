@@ -120,7 +120,6 @@ static struct {
     struct { const void* base; uint32_t row_bytes, box_rows; uint64_t rows; int swz; CUtensorMap map; } tmaps[16];
     int n_tmaps, tmap_next;
     unsigned warned_store_votes;     /* one warning per kernel and process */
-    int host_path_default;           /* host-call path for pinned buffers: 0 = staged, 1 = hybrid, 2 = zero-copy */
     const char* last_host_path;      /* "staged" | "hybrid" | "zerocopy" | "row-blocks" | "one-shot": what the last coast_run_host did */
 } G;
 
@@ -293,7 +292,6 @@ static int init_impl(int device) {
     }
     p_cuDeviceGetAttribute(&G.sm_count, CU_DEVICE_ATTRIBUTE_MULTIPROCESSOR_COUNT, G.dev);
     numa_bind_to_gpu();
-    G.host_path_default = 0;        /* measured r02 (profiles/r02_e2e_zero_copy_experiment.md) */
     r = p_cuModuleLoadData(&G.mod, coast_kernels_cubin);
     if (r != CUDA_SUCCESS) { p_cuDevicePrimaryCtxRelease_v2(G.dev); return drv_fail(r, "cuModuleLoadData(sm_100a cubin)"); }
     DRV(p_cuMemAlloc_v2(&G.counters, XMR_CTR_COUNT * sizeof(uint64_t)));
@@ -500,26 +498,16 @@ static int launch_gemm_tf32(const coast_launch_desc* d, xmr_args* a, int inj, CU
     unsigned GEMM_SMEM = stages * (16384u + 32u * bn * 4u) + 1024u + 256u;
     /* CTA-pair kernels (xmr_gemm_tf32_pair.cuh, tcgen05 cta_group::2): 256 x BN pair tiles, each CTA stages half of B.  Bit-identical
      * to the single-CTA kernels; measured at 4096^3: unprotected 0.190 vs 0.201 ms, DWC 0.320 vs 0.328 ms, TMR 0.465 vs 0.463 ms
-     * (profiles/r02_gemm_pair_timings.txt).  Default: pairs for the unprotected and DWC kernels when the shape allows (M % 256,
-     * N % BN), the single-CTA kernel for TMR; COAST_GEMM_PAIR=0 / 1 forces one or the other for every replica count. */
+     * (profiles/r02_gemm_pair_timings.txt).  Pairs for the unprotected and DWC kernels when the shape allows (M % 256, N % BN),
+     * the single-CTA kernel for TMR. */
     unsigned b_box_chunks = 4u;
     int pair = 0;
-    { const char* e = getenv("COAST_GEMM_PAIR");
-      const unsigned pbn = d->num_clones == 1 ? 256u : 128u;
-      const int want = e && (!strcmp(e, "0") || !strcmp(e, "1")) ? e[0] == '1' : d->num_clones < 3;
-      if (want && d->M % 256u == 0 && d->N % pbn == 0 && G.sm_count >= 2) {
+    { const unsigned pbn = d->num_clones == 1 ? 256u : 128u;
+      if (d->num_clones < 3 && d->M % 256u == 0 && d->N % pbn == 0 && G.sm_count >= 2) {
           pair = 1; bn = pbn; stages = d->num_clones == 1 ? 6u : 8u; b_box_chunks = 2u;
           GEMM_SMEM = stages * (16384u + 32u * (bn / 2u) * 4u) + 1024u + 256u;
           snprintf(name, sizeof name, "xmr_gemm_tf32p_nc%u_inj%d", d->num_clones, inj);
       } }
-    { const char* g = getenv("COAST_GEMM_GROUP_M"); if (g && atoi(g) > 0 && atoi(g) < 256) a->mode = (a->mode & ~0xFFu) | (unsigned)atoi(g); }
-    /* L2 eviction priorities (A evict_last, B and C evict_first): 5 % fewer DRAM reads at 4096^3, same time (profiles/r02_gemm_l2_sweep.txt) */
-    { const char* h = getenv("COAST_GEMM_L2_HINTS"); if (!(h && !strcmp(h, "0"))) a->mode |= 0x100u; }
-    /* the unprotected kernel halves the tiles of a short last round (xmr_gemm_tf32.cuh); COAST_GEMM_TAIL_SPLIT=0 keeps whole tiles */
-    { const char* h = getenv("COAST_GEMM_TAIL_SPLIT"); if (h && !strcmp(h, "0")) a->mode |= 0x200u; }
-    /* DWC / TMR: the A operand stays in the tensor core's collector across the replicas of a k-step (tcgen05.mma collector::a::fill /
-     * use / lastuse); COAST_GEMM_KEEP_A=0 re-reads it from shared memory for every replica */
-    { const char* h = getenv("COAST_GEMM_KEEP_A"); if (h && !strcmp(h, "0")) a->mode |= 0x400u; }
     CUfunction fn; int occ = 1;
     int rc = get_fn(name, GEMM_SMEM, &fn, &occ); if (rc) return rc;
     CUtensorMap ma, mb;
@@ -564,8 +552,6 @@ static int launch_mm_tc_planes(const coast_launch_desc* d, xmr_args* a, int inj,
         void* params2[] = { &B, &pb, &k32, &n32 };
         DRV(p_cuLaunchKernel(f, (unsigned)G.sm_count * 8u, 1, 1, 256, 1, 1, 0, stream, params2, NULL));
     }
-    /* the MMAs that share an A limb keep it in the tensor core's collector (xmr_mm_tc.cuh); COAST_MM_KEEP_A=0 issues them plain */
-    { const char* h = getenv("COAST_MM_KEEP_A"); if (h && !strcmp(h, "0")) a->mode |= 0x400u; else a->mode &= ~0x400u; }
     const unsigned smem = 2u * (65536u + 4u * bn * 128u) + 1024u + 256u;
     char name[64];
     snprintf(name, sizeof name, "xmr_mm_u32_%s_nc%u_inj%d", atmem ? "tct" : "tc", nc, inj);
@@ -726,10 +712,7 @@ static int launch_impl(const coast_launch_desc* d, void* stream) {
         if (d->unit_bytes < 4 || (d->unit_bytes & 3u) || d->unit_bytes > 4096u)
             return fail(COAST_ERR_BAD_ARG, "quicksort arrays are 1..1024 int32 (unit_bytes = 4*L, got %u)", d->unit_bytes);
         block = 128; qs_scratch = 1;
-        {   /* two schedulings of the same algorithm (xmr_qsort.cuh): per-unit state machine (default) or nested loops */
-            const char* path = getenv("COAST_QSORT_PATH");
-            snprintf(name, sizeof name, "%s_nc%u_inj%d", path && !strcmp(path, "nested") ? "xmr_qsortn" : "xmr_qsort", nc, inj);
-        }
+        snprintf(name, sizeof name, "xmr_qsort_nc%u_inj%d", nc, inj);
         break;
     case COAST_K_CHSTONE_SHA:
         if (d->unit_bytes < 64u || (d->unit_bytes & 63u) || d->unit_bytes >= (1u << 29))
@@ -773,7 +756,7 @@ static int launch_impl(const coast_launch_desc* d, void* stream) {
         if (d->kernel == COAST_K_AES128) {
             pack = d->n_units % 16u == 0 ? 4u : d->n_units % 4u == 0 ? 2u : 0u;
             while (pack && (tile_rows / loads) % (1u << pack)) pack -= 2u;
-            a.mode = (a.mode & ~0xF00u) | (pack << 8);
+            a.mode = (a.mode & ~XMR_AES_ROWPACK_MASK) | (pack << XMR_AES_ROWPACK_SHIFT);
         }
         rc = encode_rows_map(&map, d->d_in, row_bytes << pack, d->n_units >> pack, (tile_rows / loads) >> pack, swz); if (rc) return rc;
         uint64_t cap = (uint64_t)G.sm_count * (unsigned)occ;
@@ -1103,7 +1086,7 @@ static int run_host_impl(const coast_launch_desc* d, coast_stats* out, int* dwc_
     /* default (measured, profiles/r02_e2e_*.json): staged -- except when the output is tiny next to the input (crc16: 2 of 64 bytes,
      * CHStone sha: 20 bytes per stream), where one zero-copy launch on pinned buffers beats the chunk pipeline (1.59 vs 2.77 ms) */
     const int tiny_out = ob * 8u <= ib;
-    const int want = hp ? (!strcmp(hp, "zerocopy") ? 2 : !strcmp(hp, "hybrid") ? 1 : 0) : (tiny_out ? 2 : G.host_path_default);
+    const int want = hp ? (!strcmp(hp, "zerocopy") ? 2 : !strcmp(hp, "hybrid") ? 1 : 0) : (tiny_out ? 2 : 0);
     CUdeviceptr zin = 0;
     if (streams_once && want && ib) zin = host_alias(d->d_in, (size_t)(d->n_units * ib));
     if (want == 2 && streams_once) {

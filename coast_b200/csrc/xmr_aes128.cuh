@@ -312,7 +312,7 @@ __device__ __forceinline__ void aes128_body(const xmr_args& a, const CUtensorMap
     const uint32_t win = smem_u32(smem_raw);                    // shared-window address of the dynamic region
     uint8_t* ring_mem = smem_raw + ((1024u - (win & 1023u)) & 1023u);
     Ring ring;
-    ring.init(ring_mem, tmap, (a.mode >> 8) & 15u);             // XMR_AES_ROWPACK: 16-byte blocks described as 64- or 256-byte rows
+    ring.init(ring_mem, tmap, (a.mode & XMR_AES_ROWPACK_MASK) >> XMR_AES_ROWPACK_SHIFT);   // 16-byte blocks described as 64- or 256-byte rows
     // per-warp queue of deferred units (INJECT, one-key kernels): {unit, fault} pairs right after the ring, still below the tables
     constexpr uint32_t Q_OFF = (Ring::SMEM_BYTES + 127u) & ~127u;
     static_assert(Q_OFF + (uint32_t)AES_WARPS * AES_QCAP * 8u + 2048u + 1024u <= AES_TAB01, "ring + queues must end below the first table window");

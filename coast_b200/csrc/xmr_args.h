@@ -28,6 +28,8 @@ typedef struct xmr_args {
 #define XMR_F_STORE_VOTES 0x8000u
 /* AES: bits 8..11 of xmr_args.mode = log2 of the blocks per tensor-map row (the host describes the dense 16-byte blocks as
  * 64- or 256-byte rows when the count allows) */
+#define XMR_AES_ROWPACK_SHIFT 8u
+#define XMR_AES_ROWPACK_MASK  (15u << XMR_AES_ROWPACK_SHIFT)
 
 /* counter slots (mirror coast_stats) */
 #define XMR_CTR_ERRORS   0

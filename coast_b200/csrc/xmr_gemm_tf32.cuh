@@ -23,9 +23,10 @@
 // r02: an SS-mode kind::tf32 MMA of 128 x 128 x 8 reads 8 KiB of operands from shared memory for 64 tensor-pipe cycles =
 // 128 B/clk, exactly the SM's shared-memory bandwidth -- the r01 kernels were shared-memory-read bound (ncu: tensor pipe
 // 70 % unprotected).  Two remedies, chosen per replica count (Geom<NC>):
-//   NC >= 2 : (tried) the A tile of a stage copied ONCE from shared memory into TMEM (tcgen05.cp, 4 x 128x256b) with the NC
-//             replica MMAs of every k-step reading A from TMEM (TS mode): shared-memory reads drop from 128 to 85 (TMR) /
-//             96 (DWC) B/clk -- and the time does not move (Geom::ATMEM), so these kernels are tensor-pipe bound.
+//   NC >= 2 : the NC replica MMAs of a k-step keep A in the tensor core's collector (tc_mma_tf32_col): shared-memory reads drop
+//             from 128 to 85 (TMR) / 96 (DWC) B/clk.  Staging A in TMEM instead (tcgen05.cp + TS-mode MMAs) reads as little and
+//             was measured no faster (B200, 4096^3: TMR 0.498 vs 0.495 ms; DWC 0.354 ms): the replicated MMAs are bound by the
+//             tensor pipe itself (830 TF/s issued = 96 % of the measured cuBLAS-derived TF32 peak), not by shared-memory reads.
 //   NC == 1 : tile 128 x 256 (MMA N = 256: 12 KiB per 128 cycles = 96 B/clk) with TWO accumulator buffers, so the epilogue
 //             of tile i overlaps the main loop of tile i+1.
 #pragma once
@@ -43,21 +44,15 @@ template <int NC, bool WIDE = (NC == 1)> struct Geom {         // WIDE: 128 x 25
     static constexpr int BN = WIDE ? 256 : 128;
     static constexpr int STAGES = WIDE ? 4 : 6;
     static constexpr int ACC_BUFS = NC == 3 ? 1 : 2;             // accumulator sets: double-buffered when TMEM allows (1 x 256 x 2, 2 x 128 x 2 = 512 columns)
-    // Staging A in TMEM (tcgen05.cp + TS-mode MMAs) is built and bit-identical, but measured no faster on the B200 (r02 call 2,
-    // 4096^3: TMR 0.498 ms vs 0.495 ms with shared-memory operands; DWC 0.354 ms): the replicated MMAs are bound by the tensor
-    // pipe itself (830 TF/s issued = 96 % of the measured cuBLAS-derived TF32 peak), not by shared-memory reads.  Off.
-    static constexpr bool ATMEM = false;
     static constexpr uint32_t B_STAGE = BK * BN * 4;              // laid out [BN/32 chunks][BK rows][128 B]
     static constexpr uint32_t ACC_COLS = (uint32_t)NC * BN * ACC_BUFS;
-    static constexpr uint32_t A_COLS = ATMEM ? BK : 0;            // one tf32 per 32-bit column
-    static_assert(ACC_COLS + A_COLS <= TMEM_COLS, "TMEM budget");
+    static_assert(ACC_COLS <= TMEM_COLS, "TMEM budget");
     static constexpr uint32_t SMEM_BYTES = STAGES * (A_STAGE + B_STAGE) + 1024 /*align slack*/ + 256 /*barriers*/;
     // Instruction descriptor: c_format F32 (1) [4,6), a/b_format TF32 (2) [7,10)/[10,13), a_major K (0) [15], b_major MN (1) [16]
     // (B is row-major K x N: N contiguous), N>>3 [17,23), M>>4 [24,29)
     static constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | (0u << 15) | (1u << 16) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 };
-constexpr uint32_t GROUP_M_DEFAULT = 16;             // tile rasterisation: 16 tile-rows per group, column-major inside
-constexpr uint32_t GROUP_M = GROUP_M_DEFAULT;        // (xmr_mm_tc.cuh uses the fixed value)
+constexpr uint32_t GROUP_M = 16;                     // tile rasterisation: 16 tile-rows per group, column-major inside
 
 // Persistent CTAs take tiles blockIdx.x, +grid, ...; consecutive tile ids therefore run concurrently.  Row-major ids
 // make one wave touch ~5 A row-blocks and ALL of B (ncu r01: 489 MB read for 134 MB of operands); grouping 16 tile-rows
@@ -75,8 +70,8 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m
         "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
         ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
-// L2 eviction-priority hints (r02 experiment, xmr_args.mode bit 8): with one 32-tile-row group the whole of A (64 MiB at 4096^3)
-// should stay in the 126 MB L2 while B streams through and C is written once -- A loads evict_last, B loads and C stores evict_first.
+// L2 eviction-priority hints: A loads evict_last, B loads and C stores evict_first, so A stays in the 126 MB L2 while B streams
+// through and C is written once (5 % fewer DRAM reads at 4096^3, same time: profiles/r02_gemm_l2_sweep.txt).
 __device__ __forceinline__ uint64_t l2_policy_evict_last() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p)); return p; }
 __device__ __forceinline__ uint64_t l2_policy_evict_first() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p)); return p; }
 __device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint64_t pol) {
@@ -124,17 +119,6 @@ __device__ __forceinline__ void tc_mma_tf32_col(uint32_t d_tmem, uint64_t a_desc
     else
         tc_mma_tf32(d_tmem, a_desc, b_desc, idesc, accumulate);
 }
-// A operand from TMEM (128 lanes x 8 columns = 128 rows x 8 tf32 of K), B from shared memory
-__device__ __forceinline__ void tc_mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// shared memory (matrix descriptor, 128 rows x 256 bits) -> TMEM (128 lanes x 8 columns); SASS UTCCP
-__device__ __forceinline__ void tc_cp_a_128x256b(uint32_t taddr, uint64_t s_desc) {
-    asm volatile("tcgen05.cp.cta_group::1.128x256b [%0], %1;" ::"r"(taddr), "l"(s_desc) : "memory");
-}
 // 32 lanes x 32 consecutive fp32 columns: thread = TMEM lane (row), registers = columns
 __device__ __forceinline__ void tc_ld_32x32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile(
@@ -167,7 +151,7 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes
 // TMEM -> registers, (inject), vote with the reference's select voter / `fcmp oeq`, count, ONE store of the voted row segment.
 template <int NC, bool INJECT>
 __device__ __forceinline__ void epilogue_cols(const xmr_args& a, Tally& tally, uint32_t lane_addr, uint32_t rep_stride, uint32_t row, uint32_t n0,
-                                              int c_begin, int c_end, bool hints, uint64_t pol_c) {
+                                              int c_begin, int c_end, uint64_t pol_c) {
     const uint32_t flags = a.flags;
     const bool majority = flags & COAST_F_MAJORITY_D;
     float* C = static_cast<float*>(a.out);
@@ -204,8 +188,7 @@ __device__ __forceinline__ void epilogue_cols(const xmr_args& a, Tally& tally, u
                 o[e] = vote;
                 tally.unit_exit<NC>(bad, 1u, flags, a.unit_base + local0 + j + e);
             }
-            if (hints) st_v4_hint(dst + j, make_uint4(o[0], o[1], o[2], o[3]), pol_c);
-            else *reinterpret_cast<uint4*>(dst + j) = make_uint4(o[0], o[1], o[2], o[3]);
+            st_v4_hint(dst + j, make_uint4(o[0], o[1], o[2], o[3]), pol_c);
         }
     }
 }
@@ -228,22 +211,19 @@ __device__ __forceinline__ void gemm_body(const xmr_args& a, const CUtensorMap* 
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t tiles_n = a.N / BN, tiles_m = a.M / BM, n_tiles = tiles_m * tiles_n, kblocks = a.K / BK;
-    const uint32_t group_m = (a.mode & 0xFFu) ? (a.mode & 0xFFu) : GROUP_M_DEFAULT;
-    const bool hints = (a.mode & 0x100u) != 0;
-    const bool keep_a = (a.mode & 0x400u) == 0;               // A-operand collector reuse across the replicas (COAST_GEMM_KEEP_A=0 clears it)
     // Wave quantisation (WIDE only): 512 tiles on 148 CTAs are 3.46 rounds = 4 rounds of time.  When the last, partial round holds at
     // most grid/2 tiles, each of them is split into two 128 x 128 halves (MMA N = 128, one TMA of B instead of two), so the tail costs
     // half a round: virtual tile ids [0, sched_full) are whole tiles, [sched_full, n_virtual) are halves (two consecutive ids per tile).
     uint32_t sched_full = n_tiles, n_virtual = n_tiles;
     if (WIDE) {
         const uint32_t whole = (n_tiles / gridDim.x) * gridDim.x, rem = n_tiles - whole;
-        if (rem && 2u * rem <= gridDim.x && !(a.mode & 0x200u)) { sched_full = whole; n_virtual = whole + 2u * rem; }
+        if (rem && 2u * rem <= gridDim.x) { sched_full = whole; n_virtual = whole + 2u * rem; }
     }
     auto decode = [&](uint32_t v, uint32_t& tm, uint32_t& n_off, uint32_t& bn_t) {
         uint32_t w = v, h = 0, tn;
         bn_t = BN;
         if (v >= sched_full) { w = sched_full + ((v - sched_full) >> 1); h = (v - sched_full) & 1u; bn_t = BN / 2; }
-        tile_coords(w, tiles_m, tiles_n, group_m, tm, tn);
+        tile_coords(w, tiles_m, tiles_n, GROUP_M, tm, tn);
         n_off = tn * BN + h * (BN / 2);
     };
 
@@ -261,7 +241,6 @@ __device__ __forceinline__ void gemm_body(const xmr_args& a, const CUtensorMap* 
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    const uint32_t tmem_a = tmem_base + G::ACC_COLS;            // ATMEM: the staged A tile of the current stage
 
     if (warp == 0 && lane == 0) {
         // ===== TMA producer =====
@@ -276,13 +255,9 @@ __device__ __forceinline__ void gemm_body(const xmr_args& a, const CUtensorMap* 
                 const uint32_t s = it % STAGES, ph = (it / STAGES) & 1u;
                 mbar_wait(&empty[s], ph ^ 1u);
                 mbar_arrive_expect_tx(&full[s], A_STAGE + bn_t * BK * 4u);
-                if (hints) tma_load_2d_hint(sA + s * A_STAGE, map_a, &full[s], (int)(kb * BK), m0, pol_a);
-                else tma_load_2d(sA + s * A_STAGE, map_a, &full[s], (int)(kb * BK), m0);             // box {32 k, 128 m}
-                for (int c = 0; c < b_loads; ++c) {
-                    uint8_t* dst = sB + s * B_STAGE + c * (4 * BK * 128);
-                    if (hints) tma_load_3d_hint(dst, map_b, &full[s], 0, (int)(kb * BK), n0 / 32 + 4 * c, pol_b);
-                    else tma_load_3d(dst, map_b, &full[s], 0, (int)(kb * BK), n0 / 32 + 4 * c);
-                }
+                tma_load_2d_hint(sA + s * A_STAGE, map_a, &full[s], (int)(kb * BK), m0, pol_a);         // box {32 k, 128 m}
+                for (int c = 0; c < b_loads; ++c)
+                    tma_load_3d_hint(sB + s * B_STAGE + c * (4 * BK * 128), map_b, &full[s], 0, (int)(kb * BK), n0 / 32 + 4 * c, pol_b);
             }
         }
     } else if (warp == 1) {
@@ -308,28 +283,19 @@ __device__ __forceinline__ void gemm_body(const xmr_args& a, const CUtensorMap* 
                     // B: MN-major, 32B-atom swizzle: atom = 4 k-rows x 128 B (512 B, SBO); N chunks BK*128 B apart (LBO);
                     // one UMMA_K = 8 k-rows = 1024 B further down the chunk
                     const uint64_t db0 = smem_desc(smem_u32(sB + s * B_STAGE), BK * 128, 512, SWZ_128B_BASE32B);
-                    if (G::ATMEM) {   // tcgen05.cp and tcgen05.mma execute in issue order: this copy cannot overtake the MMAs still reading stage it-1
-#pragma unroll
-                        for (int k = 0; k < BK / UMMA_K; ++k)
-                            tc_cp_a_128x256b(tmem_a + k * UMMA_K, da0 + (uint64_t)((k * UMMA_K * 4) >> 4));
-                    }
 #pragma unroll
                     for (int k = 0; k < BK / UMMA_K; ++k) {
                         const uint64_t da = da0 + (uint64_t)((k * UMMA_K * 4) >> 4), db = db0 + (uint64_t)((k * 1024) >> 4);
                         const uint32_t acc = (kb | (uint32_t)k) ? 1u : 0u;
-                        if (G::ATMEM) {
-#pragma unroll
-                            for (int r = 0; r < NC; ++r) tc_mma_tf32_ts(acc0 + r * BN, tmem_a + k * UMMA_K, db, idesc, acc);
-                        } else if (NC == 1 || !keep_a) {
-#pragma unroll
-                            for (int r = 0; r < NC; ++r) tc_mma_tf32(acc0 + r * BN, da, db, idesc, acc);
+                        if (NC == 1) {
+                            tc_mma_tf32(acc0, da, db, idesc, acc);
                         } else {                                // A stays in the collector across the replicas of this k-step
                             tc_mma_tf32_col<1>(acc0, da, db, idesc, acc);
                             if (NC == 3) tc_mma_tf32_col<2>(acc0 + BN, da, db, idesc, acc);
                             tc_mma_tf32_col<3>(acc0 + (NC - 1) * BN, da, db, idesc, acc);
                         }
                     }
-                    tc_commit(&empty[s]);                       // smem slot free once these MMAs (and the copy) retire
+                    tc_commit(&empty[s]);                       // smem slot free once these MMAs retire
                 }
                 __syncwarp();
             }
@@ -352,7 +318,7 @@ __device__ __forceinline__ void gemm_body(const xmr_args& a, const CUtensorMap* 
             tc_fence_after();
             const uint32_t row = m0 + q * 32 + lane;
             const uint32_t lane_addr = tmem_base + buf * (uint32_t)(NC * BN) + ((uint32_t)(q * 32) << 16);
-            epilogue_cols<NC, INJECT>(a, tally, lane_addr, (uint32_t)BN, row, n0, half * (int)(bn_t / 2), (half + 1) * (int)(bn_t / 2), hints, pol_c);
+            epilogue_cols<NC, INJECT>(a, tally, lane_addr, (uint32_t)BN, row, n0, half * (int)(bn_t / 2), (half + 1) * (int)(bn_t / 2), pol_c);
             tc_fence_before();
             mbar_arrive(&tmem_empty[buf]);                      // EPI_THREADS arrivals release this accumulator set
         }

@@ -9,7 +9,7 @@
 //     DWC          256 x 128           : 24 KiB per 512 cycles         = 48 B/clk/SM   (was 64), two accumulator sets (2 x 2 x 128 = 512
 //                                        TMEM columns): the epilogue of tile i overlaps the main loop of tile i+1
 //     TMR          256 x 128           : 24 KiB per 768 cycles         = 32 B/clk/SM   (was 42.7); one accumulator set as before
-// Measured (B200, 4096^3): the TMR kernel does not move (0.465 vs 0.463 ms: tensor-pipe bound), so TMR keeps the single-CTA kernel by default.
+// Measured (B200, 4096^3): the TMR kernel does not move (0.465 vs 0.463 ms: tensor-pipe bound), so TMR always runs the single-CTA kernel.
 // Everything else is the single-CTA kernel: NC accumulators per CTA in TMEM (each CTA holds its own 128 rows x BN columns x NC),
 // the same voting epilogue (epilogue_cols), the same counters and fault site, the same per-element accumulation order over K --
 // outputs are bit-identical to xmr_gemm_tf32_* (tests/test_gpu_gemm.py).
@@ -63,7 +63,6 @@ __device__ __forceinline__ void tma2_load_3d(void* smem_dst, const CUtensorMap* 
         "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], [%2], %6;"
         ::"r"(smem_u32(smem_dst)), "l"(map), "r"(bar_cluster), "r"(c0), "r"(c1), "r"(c2), "l"(pol) : "memory");
 }
-__device__ __forceinline__ uint64_t l2_policy_normal() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p)); return p; }
 template <int USAGE>                                            // A-operand collector usage, as tc_mma_tf32_col
 __device__ __forceinline__ void tc2_mma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
     if (USAGE == 1)
@@ -100,7 +99,7 @@ __device__ __forceinline__ void mbar_wait_or_trap(uint64_t* bar, uint32_t parity
 template <int NC, bool INJECT>
 __device__ __forceinline__ void gemm_pair_body(const xmr_args& a, const CUtensorMap* map_a, const CUtensorMap* map_b) {
     using G = PairGeom<NC>;
-    constexpr int BN = G::BN, BNH = G::BNH, STAGES = G::STAGES, ACC_BUFS = G::ACC_BUFS;
+    constexpr int BN = G::BN, STAGES = G::STAGES, ACC_BUFS = G::ACC_BUFS;
     constexpr uint32_t B_STAGE = G::B_STAGE;
     extern __shared__ uint8_t smem_dyn[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023u) & ~(uintptr_t)1023u);
@@ -118,15 +117,12 @@ __device__ __forceinline__ void gemm_pair_body(const xmr_args& a, const CUtensor
     const uint32_t pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
     const uint32_t tiles_n = a.N / BN, tiles_m = a.M / 256u, n_tiles = tiles_m * tiles_n, kblocks = a.K / BK;
     // rasterisation in units of 256-row pair tiles: half as many tile-rows per group as the single-CTA kernel's 128-row tiles
-    const uint32_t gm1 = (a.mode & 0xFFu) ? (a.mode & 0xFFu) : GROUP_M_DEFAULT;
-    const uint32_t group_m = gm1 > 1u ? gm1 / 2u : 1u;
-    const bool hints = (a.mode & 0x100u) != 0;
-    const bool keep_a = (a.mode & 0x400u) == 0;
+    constexpr uint32_t group_m = GROUP_M / 2u;
     // short last round (unprotected kernel): its tiles run as two 256 x 128 halves, as in the single-CTA kernel (`decode` there)
     uint32_t sched_full = n_tiles, n_virtual = n_tiles;
     if (NC == 1) {
         const uint32_t whole = (n_tiles / n_pairs) * n_pairs, rem = n_tiles - whole;
-        if (rem && 2u * rem <= n_pairs && !(a.mode & 0x200u)) { sched_full = whole; n_virtual = whole + 2u * rem; }
+        if (rem && 2u * rem <= n_pairs) { sched_full = whole; n_virtual = whole + 2u * rem; }
     }
     auto decode = [&](uint32_t v, uint32_t& tm, uint32_t& n_off, uint32_t& bn_t) {
         uint32_t w = v, h = 0, tn;
@@ -155,7 +151,7 @@ __device__ __forceinline__ void gemm_pair_body(const xmr_args& a, const CUtensor
     if (warp == 0 && lane == 0) {
         // ===== TMA producer (both CTAs): own 128 rows of A, own half of the B columns; transactions complete on the LEADER's full[s]
         uint32_t it = 0;
-        const uint64_t pol_a = hints ? l2_policy_evict_last() : l2_policy_normal(), pol_b = hints ? l2_policy_evict_first() : l2_policy_normal();
+        const uint64_t pol_a = l2_policy_evict_last(), pol_b = l2_policy_evict_first();
         for (uint32_t tile = pair; tile < n_virtual; tile += n_pairs) {
             uint32_t tm, n_off, bn_t;
             decode(tile, tm, n_off, bn_t);
@@ -194,9 +190,8 @@ __device__ __forceinline__ void gemm_pair_body(const xmr_args& a, const CUtensor
                     for (int k = 0; k < BK / UMMA_K; ++k) {
                         const uint64_t da = da0 + (uint64_t)((k * UMMA_K * 4) >> 4), db = db0 + (uint64_t)((k * 1024) >> 4);
                         const uint32_t acc = (kb | (uint32_t)k) ? 1u : 0u;
-                        if (NC == 1 || !keep_a) {
-#pragma unroll
-                            for (int r = 0; r < NC; ++r) tc2_mma_tf32<0>(acc0 + r * BN, da, db, idesc, acc);
+                        if (NC == 1) {
+                            tc2_mma_tf32<0>(acc0, da, db, idesc, acc);
                         } else {                                // A stays in the collector across the replicas of this k-step
                             tc2_mma_tf32<1>(acc0, da, db, idesc, acc);
                             if (NC == 3) tc2_mma_tf32<2>(acc0 + BN, da, db, idesc, acc);
@@ -225,7 +220,7 @@ __device__ __forceinline__ void gemm_pair_body(const xmr_args& a, const CUtensor
             tc_fence_after();
             const uint32_t row = m0 + q * 32 + lane;
             const uint32_t lane_addr = tmem_base + buf * (uint32_t)(NC * BN) + ((uint32_t)(q * 32) << 16);
-            epilogue_cols<NC, INJECT>(a, tally, lane_addr, (uint32_t)BN, row, n0, half * (int)(bn_t / 2), (half + 1) * (int)(bn_t / 2), hints, pol_c);
+            epilogue_cols<NC, INJECT>(a, tally, lane_addr, (uint32_t)BN, row, n0, half * (int)(bn_t / 2), (half + 1) * (int)(bn_t / 2), pol_c);
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(mapa_u32(smem_u32(&tmem_empty[buf]), 0));     // one arrival per warp, on the leader's barrier
@@ -250,5 +245,5 @@ __device__ __forceinline__ void gemm_pair_body(const xmr_args& a, const CUtensor
                                      const __grid_constant__ CUtensorMap map_b) {                        \
         xmr::gemm::gemm_pair_body<NC, INJ != 0>(a, &map_a, &map_b);                                      \
     }
-XMR_GEMM_PAIR_KERNEL(1, 0) XMR_GEMM_PAIR_KERNEL(2, 0) XMR_GEMM_PAIR_KERNEL(3, 0)
-XMR_GEMM_PAIR_KERNEL(1, 1) XMR_GEMM_PAIR_KERNEL(2, 1) XMR_GEMM_PAIR_KERNEL(3, 1)
+XMR_GEMM_PAIR_KERNEL(1, 0) XMR_GEMM_PAIR_KERNEL(2, 0)
+XMR_GEMM_PAIR_KERNEL(1, 1) XMR_GEMM_PAIR_KERNEL(2, 1)

@@ -137,7 +137,6 @@ __device__ __forceinline__ void body(const xmr_args& a, const CUtensorMap* map_a
         // converged code leaves one UTCIMMA + one add per MMA.
         constexpr uint32_t IDESC_U8 = IdescU8<BN>::value;
         const bool leader = elect_one();
-        const bool keep_a = (a.mode & 0x400u) == 0;             // COAST_MM_KEEP_A=0 clears it
         uint32_t it = 0, tcount = 0;
         for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++tcount) {
             mbar_wait(tmem_empty, (tcount & 1u) ^ 1u);
@@ -157,7 +156,7 @@ __device__ __forceinline__ void body(const xmr_args& a, const CUtensorMap* map_a
                             for (int k = 0; k < TBK / 32; ++k)
                                 tc_cp_128x256b(tmem_a + (i * (TBK / 32) + k) * 8, da0 + (uint64_t)((i * (TBM * TBK) + k * 32) >> 4));
                     }
-                    if (!ATMEM && keep_a) {
+                    if (!ATMEM) {
                         // Limb-major order: the (4 - i) x NC MMAs that multiply A limb i follow each other and keep that A slice in the
                         // tensor core's collector (fill ... use ... lastuse): 4 KiB of A per k-step and limb instead of per MMA.  The u8 MMA
                         // of N = BN reads 4 KiB of A + BN x 32 B of B per 16 tensor cycles -- 5x the shared-memory bandwidth without this.
@@ -192,14 +191,11 @@ __device__ __forceinline__ void body(const xmr_args& a, const CUtensorMap* map_a
 #pragma unroll
                             for (int i = 0; i <= d; ++i) {
                                 const int j = d - i;
-                                const uint64_t da = da0 + (uint64_t)((i * (TBM * TBK) + k * 32) >> 4);
                                 const uint64_t db = db0 + (uint64_t)((j * (BN * TBK) + k * 32) >> 4);
                                 const uint32_t acc = (kb | (uint32_t)k | (uint32_t)i) ? 1u : 0u;   // first MMA into S_d overwrites
 #pragma unroll
-                                for (int r = 0; r < NC; ++r) {
-                                    if (ATMEM) tc_mma_i8_ts(tmem_base + (r * 4 + d) * BN, tmem_a + (i * (TBK / 32) + k) * 8, db, IDESC_U8, acc);
-                                    else tc_mma_i8(tmem_base + (r * 4 + d) * BN, da, db, IDESC_U8, acc);
-                                }
+                                for (int r = 0; r < NC; ++r)
+                                    tc_mma_i8_ts(tmem_base + (r * 4 + d) * BN, tmem_a + (i * (TBK / 32) + k) * 8, db, IDESC_U8, acc);
                             }
                         }
                     }

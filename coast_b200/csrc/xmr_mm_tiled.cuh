@@ -35,7 +35,7 @@ __device__ __forceinline__ void body(const xmr_args& a) {
     uint32_t* ex = smem;                        // epilogue: [NC-1][64][VT], reuses the operand buffers (64 KiB)
     const int tid = threadIdx.x, r = tid / VT, vt = tid % VT;
     const int tx = vt & 15, ty = vt >> 4;        // micro-tile: rows {ty*4+i, 32+ty*4+i}, cols {tx*4+j, 64+tx*4+j}
-    const uint32_t M = a.M, N = a.N, K = a.K;
+    const uint32_t N = a.N, K = a.K;
     const uint32_t tiles_n = N / BN;
     const uint32_t m0 = (blockIdx.x / tiles_n) * BM, n0 = (blockIdx.x % tiles_n) * BN;
     const uint32_t* __restrict__ A = static_cast<const uint32_t*>(a.in);

@@ -21,132 +21,6 @@ namespace xmr {
 
 constexpr int QS_MAX = 1024;
 
-// ---- variant 1 (COAST_QSORT_PATH=nested): the nested loops of :121-136 as written; units wait for each other at loop exits
-template <int NC>
-struct QsVote {
-    uint32_t gmask; int base; bool majority, leader;
-    uint32_t ndis = 0, syncs = 0;                               // disagreeing branch votes, executed sync points
-    // all NC lanes of the group call this together; every lane gets the same voted condition
-    __device__ __forceinline__ bool operator()(bool c) {
-        syncs++;
-        if (NC == 1) return c;
-        const int c0 = __shfl_sync(gmask, (int)c, base), c1 = __shfl_sync(gmask, (int)c, base + 1);
-        if (NC == 2) { if (c0 != c1 && leader) ndis++; return c0; }
-        const int c2 = __shfl_sync(gmask, (int)c, base + 2);
-        const bool c01 = c0 == c1, c02 = c0 == c2;
-        if (!(c01 && c02) && leader) ndis++;
-        return majority ? ((c0 & c1) | (c0 & c2) | (c1 & c2)) : (c01 ? c0 : c2);
-    }
-};
-
-template <int NC, bool INJECT>
-__device__ __forceinline__ void qsort_nested_body(const xmr_args& a) {
-    constexpr int UPW = Lanes<NC>::kUnitsPerWarp;
-    const int lane = threadIdx.x & 31;
-    const bool spare = NC == 3 && lane >= 30;                   // the two idle TMR lanes take no part in group shuffles
-    const int u = spare ? 0 : lane / NC, r = spare ? 0 : lane % NC, base = u * NC;
-    const uint32_t gmask = spare ? 0u : (((1u << NC) - 1u) << base);
-    const unsigned long long gwarp = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const unsigned long long nwarps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
-    const unsigned long long n_wtiles = (a.n_units + UPW - 1) / UPW;
-    const uint32_t L = a.unit_bytes >> 2;
-    Tally tally(a);
-    int32_t* const Au = static_cast<int32_t*>(const_cast<void*>(a.aux)) + (gwarp * 32ull + (unsigned)base) * L;   // this unit's NC x L slot
-    auto at = [&](uint32_t e) -> int32_t& { return Au[e * NC + (uint32_t)r]; };                  // element e of this replica
-    uint32_t stack[QS_MAX];                                     // (off << 16) | len, len <= 1024 needs 11 bits
-    for (unsigned long long wt = gwarp; wt < n_wtiles; wt += nwarps) {
-        const unsigned long long local = wt * UPW + u;
-        const bool valid = !spare && local < a.n_units;
-        if (valid) {
-            const int32_t* src = static_cast<const int32_t*>(a.in) + local * L;
-            for (uint32_t e = 0; e < L; ++e) at(e) = __ldg(src + e);
-            uint32_t fsite = 0xFFFFFFFFu, fmask = 0u;
-            if (INJECT) {
-                Fault f = fault_for_unit(a, NC, local, [](uint32_t) { return 32u; });
-                if (f.active) {
-                    if (r == 0) tally.injected++;
-                    if ((int)f.replica == r) { fsite = f.site; fmask = 1u << f.bit; }
-                }
-                if (fsite >= 32u * L && fsite != 0xFFFFFFFFu) at(fsite - 32u * L) ^= (int32_t)fmask;
-            }
-            QsVote<NC> vote{gmask, base, (a.flags & COAST_F_MAJORITY_D) != 0, r == 0};
-            uint32_t ev = 0;
-            int sp = 0;
-            stack[sp++] = L;                                    // off = 0
-            while (sp > 0) {
-                const uint32_t top = stack[--sp], off = top >> 16, len = top & 0xFFFFu;
-                vote.syncs++;                                   // `if (len < 2) return;` (:122) -- indices always agree
-                if (len < 2) continue;
-                const int32_t pivot = at(off + len / 2);         // :123
-                int32_t i = 0, j = (int32_t)len - 1;
-                for (;; i++, j--) {                             // :125
-                    for (;;) {                                  // while (at(i) < pivot) i++;   :126
-                        int32_t v = at(off + i);
-                        if (INJECT && fsite == ev) v ^= (int32_t)fmask;
-                        ++ev;
-                        bool c = v < pivot;
-                        if (i >= (int32_t)len - 1) c = false;   // trap guard: a mis-steered scan stops at the partition edge
-                        if (!vote(c)) break;
-                        i++;
-                    }
-                    for (;;) {                                  // while (at(j) > pivot) j--;   :127
-                        int32_t v = at(off + j);
-                        if (INJECT && fsite == ev) v ^= (int32_t)fmask;
-                        ++ev;
-                        bool c = v > pivot;
-                        if (j <= 0) c = false;
-                        if (!vote(c)) break;
-                        j--;
-                    }
-                    vote.syncs++;                               // if (i >= j) break;   :128
-                    if (i >= j) break;
-                    const int32_t t = at(off + i); at(off + i) = at(off + j); at(off + j) = t;   // :129-131, own copy
-                }
-                if (i < 1) i = 1;
-                if (i > (int32_t)len - 1) i = (int32_t)len - 1;
-                stack[sp++] = ((off + (uint32_t)i) << 16) | (len - (uint32_t)i);   // quick_sort(A + i, len - i)  :135 (later)
-                stack[sp++] = (off << 16) | (uint32_t)i;                            // quick_sort(A, i)            :134 (first)
-            }
-            // SoR exit: one vote per stored element
-            int32_t* dst = static_cast<int32_t*>(a.out) + local * L;
-            uint32_t bad = 0;
-            for (uint32_t e = 0; e < L; ++e) {
-                const int32_t x = at(e);
-                int32_t v = x;
-                if (NC >= 2) {
-                    const int32_t r1 = __shfl_sync(gmask, x, base + 1);
-                    const int32_t r0 = __shfl_sync(gmask, x, base);
-                    if (NC == 2) { bad += r0 != r1; v = r0; }
-                    else {
-                        const int32_t r2 = __shfl_sync(gmask, x, base + 2);
-                        const bool c01 = r0 == r1, c02 = r0 == r2;
-                        v = (a.flags & COAST_F_MAJORITY_D) ? ((r0 & r1) | (r0 & r2) | (r1 & r2)) : (c01 ? r0 : r2);
-                        bad += (c01 && c02) ? 0u : 1u;
-                    }
-                }
-                if (r == 0) dst[e] = v;
-            }
-            if (r == 0) {
-                const unsigned long long gunit = a.unit_base + local;
-                if (NC == 3) {
-                    if (a.flags & COAST_F_COUNT_ERRORS_D) {
-                        tally.errors += bad + vote.ndis;
-                        if (a.flags & COAST_F_COUNT_SYNCS_D) tally.syncs += vote.syncs + L;
-                    }
-                } else if (NC == 2) {
-                    tally.dwc += (bad || vote.ndis) ? 1u : 0u;
-                }
-                const uint32_t dis = bad + vote.ndis;
-                if (NC > 1 && dis && gunit < tally.first) tally.first = gunit;
-                if (tally.status) tally.status[local] = (unsigned char)(NC > 1 ? (dis > 255u ? 255u : dis) : 0u);
-            }
-        }
-        __syncwarp();
-    }
-    tally.flush(a.counters);
-}
-
-
 // Execution scheme: a per-unit STATE MACHINE stepped by one uniform warp loop.  Written as the nested loops of :121-136,
 // the units of a warp wait for each other at every loop exit (scan lengths and partition sizes differ wildly between
 // arrays), which left ~1 lane group in 10 busy (r01: 16 ms TMR, issue-bound on serialised paths).  Here every iteration
@@ -297,10 +171,5 @@ __device__ __forceinline__ void qsort_body(const xmr_args& a) {
 #define XMR_QSORT_KERNEL(NC, INJ)                                                                        \
     extern "C" __global__ void __launch_bounds__(128)                                                    \
     xmr_qsort_nc##NC##_inj##INJ(const __grid_constant__ xmr_args a) { xmr::qsort_body<NC, INJ != 0>(a); }
-#define XMR_QSORT_NESTED_KERNEL(NC, INJ)                                                                 \
-    extern "C" __global__ void __launch_bounds__(128)                                                    \
-    xmr_qsortn_nc##NC##_inj##INJ(const __grid_constant__ xmr_args a) { xmr::qsort_nested_body<NC, INJ != 0>(a); }
-XMR_QSORT_NESTED_KERNEL(1, 0) XMR_QSORT_NESTED_KERNEL(2, 0) XMR_QSORT_NESTED_KERNEL(3, 0)
-XMR_QSORT_NESTED_KERNEL(1, 1) XMR_QSORT_NESTED_KERNEL(2, 1) XMR_QSORT_NESTED_KERNEL(3, 1)
 XMR_QSORT_KERNEL(1, 0) XMR_QSORT_KERNEL(2, 0) XMR_QSORT_KERNEL(3, 0)
 XMR_QSORT_KERNEL(1, 1) XMR_QSORT_KERNEL(2, 1) XMR_QSORT_KERNEL(3, 1)

@@ -1,4 +1,4 @@
-// xmr_util.cuh -- small service kernels of the runtime (counter reset/snapshot, synthetic input).
+// xmr_util.cuh -- small service kernels of the runtime (counter reset, synthetic input).
 #pragma once
 #include "xmr_common.cuh"
 
@@ -27,9 +27,6 @@ xmr_fill_philox(uint32_t* __restrict__ dst, unsigned long long n_words, unsigned
 
 extern "C" __global__ void xmr_counters_reset(unsigned long long* ctr) {
     if (threadIdx.x < XMR_CTR_COUNT) ctr[threadIdx.x] = threadIdx.x == XMR_CTR_FIRST ? ~0ull : 0ull;
-}
-extern "C" __global__ void xmr_counters_copy(const unsigned long long* ctr, unsigned long long* dst) {
-    if (threadIdx.x < XMR_CTR_COUNT) dst[threadIdx.x] = ctr[threadIdx.x];
 }
 
 // One record per SM that gets a CTA: {clock64(), %globaltimer [ns]} at out[2 * smid ..].  Two probes around a region give the

@@ -40,20 +40,22 @@ def test_sm100a_cubin_is_embedded(built_lib):
     assert cubin[:4] == b"\x7fELF" and cubin in blob
 
 
-def test_every_kernel_the_host_code_can_name_is_in_the_cubin(built_lib):
-    """coast_rt.c builds kernel names with snprintf; a typo would only show up as a launch failure on a GPU box"""
+def test_cubin_kernels_are_exactly_those_the_host_code_can_name(built_lib):
+    """coast_rt.c builds kernel names with snprintf; a typo would only show up as a launch failure on a GPU box.  Conversely, every
+    kernel in the cubin is one the host code can launch: nothing is built that no path reaches."""
     import itertools
     import re
     import subprocess
     src = open(os.path.join(ROOT, "coast_b200", "csrc", "coast_rt.c")).read()
     fmts = set(re.findall(r'"(xmr_[A-Za-z0-9_%]+)"', src))
-    stems = {"xmr_qsort", "xmr_qsortn", "xmr_aes128_enc", "xmr_aes128_dec", "xmr_aes128_enck", "xmr_aes128_deck",
+    stems = {"xmr_aes128_enc", "xmr_aes128_dec", "xmr_aes128_enck", "xmr_aes128_deck",
              "xmr_chaes_enc", "xmr_chaes_dec"}               # stems of a "%s_nc%u_inj%d"
     assert stems <= fmts
     fmts = (fmts - stems) | {s + "_nc%u_inj%d" for s in stems}
     names = set()
     for f in fmts:
-        opts = [["tc", "tct"] if tok == "%s" else ["1", "2", "3"] if tok == "%u" else ["0", "1"] for tok in re.findall(r"%[sud]", f)]
+        ncs = ["1", "2"] if f.startswith("xmr_gemm_tf32p_") else ["1", "2", "3"]     # CTA pairs for nc < 3 only
+        opts = [["tc", "tct"] if tok == "%s" else ncs if tok == "%u" else ["0", "1"] for tok in re.findall(r"%[sud]", f)]
         for combo in itertools.product(*opts):
             it = iter(combo)
             names.add(re.sub(r"%[sud]", lambda m: next(it), f))
@@ -61,6 +63,7 @@ def test_every_kernel_the_host_code_can_name_is_in_the_cubin(built_lib):
                           capture_output=True, text=True).stdout
     have = set(re.findall(r"\.text\.(xmr_\w+)", sass))
     assert len(names) > 80 and not (names - have), sorted(names - have)
+    assert not (have - names), sorted(have - names)
 
 
 @pytest.mark.parametrize("s,nc,fl", [

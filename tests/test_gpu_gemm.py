@@ -50,60 +50,67 @@ def test_gemm_tf32_matches_truncated_fp64_reference(rt, oracle, M, N, K):
     assert np.abs(o.view(np.float32).reshape(M, N) - outs[3]).max() <= 2e-6 * K
 
 
+def check_faults_against_clean(rt, oracle, A, B, clean, seed, p):
+    """DWC and TMR under a Bernoulli fault plan: TMR votes every fault out (the clean bits); DWC stores replica 0, so its output
+    differs from the clean one in exactly the bits the oracle flips in replica 0; counters equal the oracle's"""
+    import coast_b200 as cb
+    M, K = A.shape
+    N = B.shape[1]
+    plan = cb.FaultPlan(mode=cb.PLAN_BERNOULLI, seed=seed, p=p)
+    got, want = {}, {}
+    for nc in (2, 3):
+        got[nc], st = run(rt, nc, A, B, plan=plan)
+        want[nc], so = oracle.run(oracle.K_GEMM_TF32, nc, A, M * N, M=M, N=N, K=K, aux=B, flags=3,
+                                  plan=oracle.make_plan(oracle.PLAN_BERNOULLI, seed=seed, p=p))
+        assert st.as_dict() == so and st.injected > 0, (nc, st.as_dict(), so)
+    assert got[3].tobytes() == clean.tobytes()
+    flipped = want[2].view(np.uint32) ^ want[3].view(np.uint32)       # the oracle's TMR output is its clean output
+    assert ((got[2].view(np.uint32) ^ clean.view(np.uint32)).ravel() == flipped.ravel()).all() and flipped.any()
+
+
 @pytest.mark.parametrize("M,N,K", [(2432, 2048, 64), (2560, 2048, 96)])
-def test_gemm_unprotected_tail_split_is_bit_identical(rt, oracle, M, N, K, monkeypatch):
-    """152 / 160 tiles of 128 x 256 on 148 CTAs: the 4 / 12 tiles of the short last round run as 128 x 128 halves (xmr_gemm_tf32.cuh,
-    `decode`); every element accumulates over K in the same order, so the output equals the whole-tile schedule's and the TMR kernel's"""
+def test_gemm_unprotected_tail_split_is_bit_identical(rt, oracle, M, N, K):
+    """152 single-CTA 128 x 256 tiles on 148 CTAs / 80 pair tiles of 256 x 256 on 74 CTA pairs: the 4 / 6 tiles of the short last round
+    run as halves (`decode` in xmr_gemm_tf32*.cuh); every element accumulates over K in the same order, so the output equals the TMR
+    kernel's, whose single-CTA 128 x 128 schedule has no split"""
     A, B = operands(oracle, M, N, K, seed=12)
     split, _ = run(rt, 1, A, B)
-    monkeypatch.setenv("COAST_GEMM_TAIL_SPLIT", "0")
-    whole, _ = run(rt, 1, A, B)
-    monkeypatch.delenv("COAST_GEMM_TAIL_SPLIT")
     tmr, st = run(rt, 3, A, B)
-    assert split.tobytes() == whole.tobytes() == tmr.tobytes() and st.errors_corrected == 0
+    assert split.tobytes() == tmr.tobytes() and st.errors_corrected == 0
     ref = tf32(A).astype(np.float64) @ tf32(B).astype(np.float64)
     assert np.abs(split - ref).max() <= 2e-6 * K
 
 
 @pytest.mark.parametrize("M,N,K", [(256, 256, 32), (256, 256, 256), (512, 768, 96), (1024, 512, 2048), (2560, 4096, 64)])
-def test_gemm_cta_pair_kernels_are_bit_identical_to_the_single_cta_kernels(rt, oracle, M, N, K, monkeypatch):
-    """xmr_gemm_tf32p_* (tcgen05 cta_group::2, 256 x BN pair tiles, each CTA stages half of B): same operands, same accumulation order
-    over K per element -> the same bits as xmr_gemm_tf32_*, for every replica count, with and without injected faults, same counters"""
-    import coast_b200 as cb
+def test_gemm_cta_pair_kernels_are_bit_identical_to_the_single_cta_kernels(rt, oracle, M, N, K):
+    """the unprotected and DWC kernels run on CTA pairs (xmr_gemm_tf32p_*, tcgen05 cta_group::2, 256 x BN pair tiles, each CTA stages
+    half of B), TMR on single CTAs (xmr_gemm_tf32_*): same operands, same accumulation order over K per element -> the same bits for
+    every replica count; with injected faults, the outputs and counters the protection promises"""
     A, B = operands(oracle, M, N, K, seed=21)
-    plan = cb.FaultPlan(mode=cb.PLAN_BERNOULLI, seed=3, p=0.01)
-    monkeypatch.setenv("COAST_GEMM_PAIR", "0")
-    single = {nc: run(rt, nc, A, B) for nc in (1, 2, 3)}
-    single_f = {nc: run(rt, nc, A, B, plan=plan) for nc in (2, 3)}
-    monkeypatch.setenv("COAST_GEMM_PAIR", "1")
-    for nc in (1, 2, 3):
+    single, _ = run(rt, 3, A, B)
+    for nc in (1, 2):
         C, st = run(rt, nc, A, B)
-        assert C.tobytes() == single[nc][0].tobytes(), (nc, np.abs(C - single[nc][0]).max())
-        assert st.as_dict() == single[nc][1].as_dict()
-    for nc in (2, 3):
-        C, st = run(rt, nc, A, B, plan=plan)
-        assert C.tobytes() == single_f[nc][0].tobytes() and st.as_dict() == single_f[nc][1].as_dict() and st.injected > 0
+        assert C.tobytes() == single.tobytes(), (nc, np.abs(C - single).max())
+        assert st.errors_corrected == st.dwc_detected == st.injected == 0
+    check_faults_against_clean(rt, oracle, A, B, single, seed=3, p=0.01)
     ref = tf32(A).astype(np.float64) @ tf32(B).astype(np.float64)
-    assert np.abs(single[1][0] - ref).max() <= 2e-6 * K
+    assert np.abs(single - ref).max() <= 2e-6 * K
 
 
-@pytest.mark.parametrize("pair", ["0", "1"])
-def test_gemm_a_operand_collector_reuse_changes_nothing(rt, oracle, pair, monkeypatch):
+@pytest.mark.parametrize("M", [384, 512])
+def test_gemm_a_operand_collector_reuse_changes_nothing(rt, oracle, M):
     """DWC / TMR: the replicas of a k-step keep A in the tensor core's collector (tcgen05.mma collector::a::fill / use / lastuse) instead
-    of re-reading it from shared memory -- same products, same accumulation order, same bits and counters, with and without faults"""
-    import coast_b200 as cb
-    M, N, K = 512, 768, 352
+    of re-reading it from shared memory -- same products, same accumulation order: the bits of the unprotected kernel, which issues
+    plain MMAs, with and without faults.  M = 384 runs DWC and TMR on single CTAs, M = 512 runs DWC on CTA pairs."""
+    N, K = 768, 352
     A, B = operands(oracle, M, N, K, seed=31)
-    plan = cb.FaultPlan(mode=cb.PLAN_BERNOULLI, seed=8, p=0.01)
-    monkeypatch.setenv("COAST_GEMM_PAIR", pair)
-    monkeypatch.setenv("COAST_GEMM_KEEP_A", "0")
-    plain = {nc: run(rt, nc, A, B, plan=plan) for nc in (2, 3)}
-    monkeypatch.delenv("COAST_GEMM_KEEP_A")
+    plain, _ = run(rt, 1, A, B)
     for nc in (2, 3):
-        C, st = run(rt, nc, A, B, plan=plan)
-        assert C.tobytes() == plain[nc][0].tobytes() and st.as_dict() == plain[nc][1].as_dict() and st.injected > 0
+        C, st = run(rt, nc, A, B)
+        assert C.tobytes() == plain.tobytes() and st.errors_corrected == st.dwc_detected == 0
+    check_faults_against_clean(rt, oracle, A, B, plain, seed=8, p=0.01)
     ref = tf32(A).astype(np.float64) @ tf32(B).astype(np.float64)
-    assert np.abs(plain[3][0] - ref).max() <= 2e-6 * K
+    assert np.abs(plain - ref).max() <= 2e-6 * K
 
 
 def test_gemm_faults_are_voted_out_and_counted(rt, oracle):

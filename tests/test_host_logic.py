@@ -191,22 +191,21 @@ def test_tf32_gemm_launch(mock_dir, tmp_path):
     assert bad["ops"][0]["rc"] != 0 and "multiples of 128" in bad["ops"][0]["err"]
 
 
-@pytest.mark.parametrize("nc,M,N,pair_env,want_name,want_grid", [
-    (1, 512, 512, None, "xmr_gemm_tf32p_nc1_inj0", 8),       # unprotected: CTA pairs, 256 x 256 pair tiles -> 4 pairs
-    (2, 512, 512, None, "xmr_gemm_tf32p_nc2_inj0", 16),      # DWC: pairs, 256 x 128
-    (3, 512, 512, None, "xmr_gemm_tf32_nc3_inj0", 16),       # TMR: single-CTA kernel by default ...
-    (3, 512, 512, "1", "xmr_gemm_tf32p_nc3_inj0", 16),       # ... pairs on request
-    (1, 512, 512, "0", "xmr_gemm_tf32_nc1_inj0", 8),         # single-CTA 128 x 256
-    (1, 384, 512, None, "xmr_gemm_tf32_nc1_inj0", 6),        # M not a multiple of 256: no pair tile
-    (1, 512, 384, None, "xmr_gemm_tf32n_nc1_inj0", 12),      # N % 256 != 0: the narrow single-CTA kernel
-    (2, 512, 384, None, "xmr_gemm_tf32p_nc2_inj0", 12),
+@pytest.mark.parametrize("nc,M,N,want_name,want_grid", [
+    (1, 512, 512, "xmr_gemm_tf32p_nc1_inj0", 8),         # unprotected: CTA pairs, 256 x 256 pair tiles -> 4 pairs
+    (2, 512, 512, "xmr_gemm_tf32p_nc2_inj0", 16),        # DWC: pairs, 256 x 128
+    (3, 512, 512, "xmr_gemm_tf32_nc3_inj0", 16),         # TMR: always the single-CTA kernel
+    (1, 384, 512, "xmr_gemm_tf32_nc1_inj0", 6),          # M not a multiple of 256: no pair tile, single-CTA 128 x 256
+    (2, 384, 512, "xmr_gemm_tf32_nc2_inj0", 12),         # ... and single-CTA 128 x 128 for DWC
+    (1, 512, 384, "xmr_gemm_tf32n_nc1_inj0", 12),        # N % 256 != 0: the narrow single-CTA kernel
+    (2, 512, 384, "xmr_gemm_tf32p_nc2_inj0", 12),
+    (2, 2048, 2048, "xmr_gemm_tf32p_nc2_inj0", 148),     # more tiles than SMs: one persistent CTA per SM
 ])
-def test_tf32_gemm_kernel_selection_pairs_and_single(mock_dir, tmp_path, nc, M, N, pair_env, want_name, want_grid):
+def test_tf32_gemm_kernel_selection_pairs_and_single(mock_dir, tmp_path, nc, M, N, want_name, want_grid):
     """which TF32 GEMM kernel a shape gets (single CTA / CTA pair, wide / narrow), with an EVEN grid for the cluster kernels and the
     B box matching what each kernel loads per TMA (64 columns for pairs, 128 for single CTAs)"""
-    env = {"COAST_GEMM_PAIR": pair_env} if pair_env is not None else None
     res, ev = run_child(mock_dir, tmp_path, [dict(op="launch", kernel=K_GEMM_TF32, nc=nc, n=M * N, M=M, N=N, K=64, in_bytes=M * 64 * 4,
-                                                  aux_bytes=64 * N * 4, out_bytes=M * N * 4, flags=3)], env_extra=env)
+                                                  aux_bytes=64 * N * 4, out_bytes=M * N * 4, flags=3)])
     assert res["ops"][0]["rc"] == 0 and not [e for e in ev if e["op"] == "error"], res
     la = [e for e in ev if e["op"] == "launch" and "_nc" in e["name"]][0]
     assert (la["name"], la["grid"], la["block"]) == (want_name, want_grid, 384) and la["smem"] <= 232448
@@ -216,21 +215,36 @@ def test_tf32_gemm_kernel_selection_pairs_and_single(mock_dir, tmp_path, nc, M, 
     assert tm[1]["box_bytes"] == 32 * 32 * 4 * (2 if "tf32p" in want_name else 4), tm[1]
 
 
-def test_gemm_tuning_switches_reach_the_kernel_as_mode_bits(mock_dir, tmp_path):
-    """COAST_GEMM_GROUP_M / _L2_HINTS / _TAIL_SPLIT / _KEEP_A (TF32) and COAST_MM_KEEP_A (integer limb kernel) are read per launch and
-    travel in xmr_args.mode: bits 0-7 group, 0x100 hints on, 0x200 tail split off, 0x400 collector reuse off"""
+def test_retired_tuning_variables_change_no_launch(mock_dir, tmp_path):
+    """the GEMM, limb-matmul and quicksort experiment switches of earlier releases are gone: with all of them set, every launch
+    (kernel, grid, block, shared memory, tensor maps, argument block) is the one made without them"""
     s = 512
-    gemm = dict(op="launch", kernel=K_GEMM_TF32, nc=3, n=s * s, M=s, N=s, K=64, in_bytes=s * 64 * 4, aux_bytes=64 * s * 4, out_bytes=s * s * 4, flags=3)
-    mm = dict(op="launch", kernel=K_MM_U32, nc=3, n=s * s, M=s, N=s, K=128, in_bytes=s * 128 * 4, aux_bytes=128 * s * 4, out_bytes=s * s * 4, flags=3)
-    res, ev = run_child(mock_dir, tmp_path, [gemm, mm], env_extra={"COAST_MM_PATH": "tc"})
-    la = [e for e in ev if e["op"] == "launch" and "_nc" in e["name"]]
-    assert [x["name"] for x in la] == ["xmr_gemm_tf32_nc3_inj0", "xmr_mm_u32_tc_nc3_inj0"]
-    assert args_of(la[0]).mode == 0x100 and args_of(la[1]).mode & 0x400 == 0
-    env = {"COAST_GEMM_GROUP_M": "8", "COAST_GEMM_L2_HINTS": "0", "COAST_GEMM_TAIL_SPLIT": "0", "COAST_GEMM_KEEP_A": "0", "COAST_MM_KEEP_A": "0",
-           "COAST_MM_PATH": "tc"}
-    res, ev = run_child(mock_dir, tmp_path, [gemm, mm], env_extra=env)
-    la = [e for e in ev if e["op"] == "launch" and "_nc" in e["name"]]
-    assert args_of(la[0]).mode == 8 | 0x200 | 0x400 and args_of(la[1]).mode & 0x400
+    gemm = dict(op="launch", kernel=K_GEMM_TF32, n=s * s, M=s, N=s, K=64, in_bytes=s * 64 * 4, aux_bytes=64 * s * 4, out_bytes=s * s * 4, flags=3)
+    ops = [dict(gemm, nc=1), dict(gemm, nc=3),
+           dict(op="launch", kernel=K_MM_U32, nc=2, n=s * s, M=s, N=s, K=128, in_bytes=s * 128 * 4, aux_bytes=128 * s * 4,
+                out_bytes=s * s * 4, flags=3),
+           dict(op="launch", kernel=K_QSORT, nc=3, n=100, unit_bytes=4 * 580, in_bytes=100 * 4 * 580, out_bytes=100 * 4 * 580, flags=3)]
+    pointers = ("inp", "out", "aux", "counters", "plan_table", "status")
+
+    def launches(env):
+        res, ev = run_child(mock_dir, tmp_path, ops, env_extra=env)
+        assert [r["rc"] for r in res["ops"]] == [0] * len(ops) and not [e for e in ev if e["op"] == "error"], res
+        log = []
+        for e in ev:
+            if e["op"] == "tmap":
+                log.append(e)
+            elif e["op"] == "launch" and "_nc" in e["name"]:
+                a = args_of(e)
+                log.append((e["name"], e["grid"], e["block"], e["smem"],
+                            [(f, getattr(a, f)) for f, _ in XmrArgs._fields_ if f not in pointers and f != "key"] + [("key", bytes(a.key))]))
+        return log
+
+    plain = launches({})
+    assert [x[0] for x in plain if isinstance(x, tuple)] == ["xmr_gemm_tf32p_nc1_inj0", "xmr_gemm_tf32_nc3_inj0", "xmr_mm_u32_tc_nc2_inj0",
+                                                             "xmr_qsort_nc3_inj0"]
+    retired = {"COAST_QSORT_PATH": "nested", "COAST_GEMM_PAIR": "1", "COAST_GEMM_GROUP_M": "8", "COAST_GEMM_L2_HINTS": "0",
+               "COAST_GEMM_TAIL_SPLIT": "0", "COAST_GEMM_KEEP_A": "0", "COAST_MM_KEEP_A": "0"}
+    assert launches(retired) == plain
 
 
 def test_quicksort_through_the_host_call_uses_one_scratch_slot_per_chunk(mock_dir, tmp_path):
